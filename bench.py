@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on host cores
+    python bench.py --gpus 1 --steps K --dump-outputs bench_outputs  # + the last timed step's results as .npy files
 
 One "step" = one QAGNN_Message_Passing.forward (k=5 GATConvE layers, modeling_qagnn.py:53-95) over one
 synthetic batch of BASELINE.json configs[1]: 64x5 = 320 sub-graphs of 200 nodes / 1000 edges per GPU,
@@ -38,7 +39,29 @@ def parse():
     ap.add_argument("--cpu-sample-graphs", type=int, default=64)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cuda-graph", action="store_true", help="launch the ~60 kernels of a step one by one")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (logits, pool_attn, gnn_out of "
+                         "rank 0) as DIR/<name>.npy in float32; the inputs are seeded, so two builds compare output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200 (the reference arm times a sample sized to the host)")
+    return args
+
+
+DUMP_LIMIT = 64 << 20  # bytes, all dumped arrays together
+
+
+def dump_outputs(dirname, arrays):
+    """Writes {name: float32 ndarray} as dirname/<name>.npy."""
+    import numpy as np
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"bench.py: the outputs take {total} bytes, more than the {DUMP_LIMIT} of --dump-outputs")
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def workload_name():
@@ -372,6 +395,12 @@ def run_b200_arm(args):
     if rank == 0:
         sampler.start()
     ms_total, _, _ = timed(step_resident, args.steps)
+    # the results of the last timed step, (logits, pool_attn, gnn_out) as DecoderStep.run returns them; the passes below
+    # run the same model on other buffers
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        dumped = {name: t.detach().float().cpu().numpy()
+                  for name, t in zip(("logits", "pool_attn", "gnn_out"), (step.logits, step.pool_attn, step.gnn_out))}
     ms_e2e = timed_e2e(runner, args.steps)
     ms_e2e_nodes = timed_e2e(runner_nodes, args.steps) if world == 1 else None
     # kernel-level pass: the same K steps launched kernel by kernel with the library's CUDA-event stage timers on the
@@ -416,6 +445,8 @@ def run_b200_arm(args):
     if rank != 0:
         finish()
         return
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, dumped)
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
         "ms_per_step": ms_step, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",

@@ -1,10 +1,12 @@
 """TEST INFRASTRUCTURE — mints tests/golden/*.pt from the reference's OWN modules.
 
-Run in the build container only (needs /root/reference):
+Needs the reference tree (oracle/ref_shim.py, QAGNN_REFERENCE_ROOT):
 
     python -m oracle.make_goldens            # writes tests/golden/*.pt
     python -m oracle.make_goldens --check    # re-mints in memory, compares with the committed files, writes nothing
     python -m oracle.make_goldens --fuzz 24  # reference vs oracle on 24 random cases that are not committed as fixtures
+    python -m oracle.make_goldens --record   # stores what the reference produced where the tests compare against it
+                                             # (tests/golden/reference_digests.json, fuzz_mp_sampled.pt)
 
 Every fixture is produced by the unmodified `GATConvE` / `QAGNN_Message_Passing` / `QAGNN`
 classes of /root/reference/modeling/modeling_qagnn.py (imported through oracle/ref_shim.py),
@@ -13,6 +15,7 @@ in eval mode, fp32, on CPU.  Inputs and weights are regenerated deterministicall
 case description, a fingerprint of the regenerated inputs, and the reference outputs.
 """
 import hashlib
+import json
 import os
 import sys
 
@@ -325,34 +328,217 @@ def check(names=None):
     return out
 
 
-def fuzz(count, tol_abs=2e-6, tol_rel=2e-5):
-    """Random small cases that are NOT committed as fixtures: the reference's own QAGNN_Message_Passing against the oracle
-    (output, node_feature_extra, first / last layer x and attention, edge_index').  Returns [(case, worst excess over the
-    tolerance)]; excess <= 0 means inside `tol_abs + tol_rel*|ref|`."""
-    torch.set_num_threads(8)
-    ref = load_reference()
+FUZZ_TOL = (2e-6, 2e-5)  # abs, rel: the oracle and the reference run the same fp32 op sequence
+
+
+def fuzz_cases(count):
+    """Random small cases outside the fixture table (1-4 graphs, 1-30 nodes, 0-80 edges, D 16-100, k 1-3, 6 / 17 / 38 edge
+    types, both weight regimes); the i-th case is the same for every `count`."""
     g = torch.Generator().manual_seed(12345)
     ri = lambda lo, hi: int(torch.randint(lo, hi + 1, (1,), generator=g))  # noqa: E731
-    results = []
+    cases = []
     for i in range(count):
         n = ri(1, 30)
         R = (38, 38, 6, 17)[ri(0, 3)]
-        case = dict(name=f"fuzz{i}", B=ri(1, 4), n=n, e=ri(0, 80), D=(16, 32, 64, 100)[ri(0, 3)], k=ri(1, 3),
-                    regime=("prod", "peaky")[ri(0, 1)], realistic=bool(ri(0, 1)) and n >= 8 and R >= 6, seed=100 + i)
-        fx = mint_mp_case(ref, case, 4, R)
-        inp = O.synth_graph_batch(case["B"], case["n"], case["e"], case["D"], R, case["seed"], case["realistic"])
-        sd = O.random_state_dict(case["k"], case["D"], 4, R, case["regime"], case["seed"])
-        out, extra, layers = O.message_passing_forward(sd, inp["H"], inp["edge_index"], inp["edge_type"], inp["node_type"],
-                                                       inp["node_score"], case["k"], 4, R, return_layers=True)
-        pairs = [(out, fx["out"]), (extra, fx["extra"])]
-        for l, want in fx["layers"].items():
-            pairs += [(layers[l]["x"], want["x"]), (layers[l]["alpha"], want["alpha"])]
-        worst = max(float(((a - b).abs() - tol_abs - tol_rel * b.abs()).max()) if a.numel() else -tol_abs for a, b in pairs)
-        results.append((dict(case, n_etype=R), worst))
+        cases.append(dict(name=f"fuzz{i}", B=ri(1, 4), n=n, e=ri(0, 80), D=(16, 32, 64, 100)[ri(0, 3)], k=ri(1, 3),
+                          regime=("prod", "peaky")[ri(0, 1)], realistic=bool(ri(0, 1)) and n >= 8 and R >= 6, seed=100 + i,
+                          n_etype=R))
+    return cases
+
+
+def _fuzz_compared(fx):
+    """The tensors a fuzz case compares, by name: output, node_feature_extra, x and attention of the first / last layer."""
+    out = {"out": fx["out"], "extra": fx["extra"]}
+    for l, layer in fx["layers"].items():
+        out[f"x[{l}]"], out[f"alpha[{l}]"] = layer["x"], layer["alpha"]
+    return out
+
+
+def fuzz_oracle(case):
+    """The oracle's side of a fuzz case: (input fingerprint, weight fingerprint, {name: tensor} as _fuzz_compared)."""
+    R = case["n_etype"]
+    inp = O.synth_graph_batch(case["B"], case["n"], case["e"], case["D"], R, case["seed"], case["realistic"])
+    sd = O.random_state_dict(case["k"], case["D"], 4, R, case["regime"], case["seed"])
+    out, extra, layers = O.message_passing_forward(sd, inp["H"], inp["edge_index"], inp["edge_type"], inp["node_type"],
+                                                   inp["node_score"], case["k"], 4, R, return_layers=True)
+    keep = [0, case["k"] - 1] if case["k"] > 1 else [0]
+    fx = {"out": out, "extra": extra, "layers": {l: layers[l] for l in keep}}
+    return (fingerprint(inp["H"], inp["edge_index"], inp["edge_type"], inp["node_type"], inp["node_score"]),
+            fingerprint(*[sd[k_] for k_ in sorted(sd) if sd[k_].dtype.is_floating_point]), _fuzz_compared(fx))
+
+
+def _excess(a, b, tol_abs, tol_rel):
+    return float(((a - b).abs() - tol_abs - tol_rel * b.abs()).max()) if a.numel() else -tol_abs
+
+
+def fuzz(count, tol_abs=FUZZ_TOL[0], tol_rel=FUZZ_TOL[1]):
+    """The reference's own QAGNN_Message_Passing against the oracle on `count` fuzz cases, every element compared.  Returns
+    [(case, worst excess over the tolerance)]; excess <= 0 means inside `tol_abs + tol_rel*|ref|`."""
+    torch.set_num_threads(8)
+    ref = load_reference()
+    results = []
+    for case in fuzz_cases(count):
+        want = _fuzz_compared(mint_mp_case(ref, case, 4, case["n_etype"]))
+        got = fuzz_oracle(case)[2]
+        results.append((case, max(_excess(got[k_], want[k_], tol_abs, tol_rel) for k_ in want)))
     return results
 
 
+# ---------------------------------------------------------------------------------------------
+# what the reference produced, stored for the tests (`--record`): content digests where the tests compare bit for bit,
+# a seeded sample of every compared tensor where they compare within a tolerance
+# ---------------------------------------------------------------------------------------------
+DIGEST_FILE = os.path.join(GOLDEN_DIR, "reference_digests.json")
+FUZZ_FILE = os.path.join(GOLDEN_DIR, "fuzz_mp_sampled.pt")
+FUZZ_COUNT = 24
+FUZZ_SAMPLES = 128  # entries kept per compared tensor
+LOADER_CASE = dict(n_records=20, seed=4, num_choice=5)
+LOADER_FIELDS = ("concept_ids", "node_type_ids", "node_scores", "adj_lengths", "edge_index", "edge_type")
+
+
+def digest(obj):
+    """sha256 over nested dicts / lists / tuples of tensors and scalars.  Equal digests: same structure, and every tensor
+    has the same dtype, shape and bits (lists and tuples count as the same)."""
+    h = hashlib.sha256()
+
+    def walk(o):
+        if isinstance(o, dict):
+            h.update(b"{")
+            for k_ in sorted(o, key=repr):
+                h.update(repr(k_).encode())
+                walk(o[k_])
+            h.update(b"}")
+        elif isinstance(o, (list, tuple)):
+            h.update(b"[%d" % len(o))
+            for x in o:
+                walk(x)
+            h.update(b"]")
+        elif torch.is_tensor(o):
+            t = o.detach().contiguous().cpu()
+            h.update(f"T{t.dtype}{tuple(t.shape)}".encode())
+            h.update(t.numpy().tobytes())
+        else:
+            h.update(repr(o).encode())
+    walk(obj)
+    return h.hexdigest()
+
+
+def records_digest(records):
+    """Digest of the content of `*.graph.adj.pk` records (qagnn_b200.data.synth_adj_pickle)."""
+    import numpy as np
+    return digest([[torch.from_numpy(r["adj"].row.astype(np.int64)), torch.from_numpy(r["adj"].col.astype(np.int64)),
+                    tuple(r["adj"].shape), torch.from_numpy(np.asarray(r["concepts"], dtype=np.int64)),
+                    torch.from_numpy(np.asarray(r["qmask"], dtype=bool)), torch.from_numpy(np.asarray(r["amask"], dtype=bool)),
+                    sorted(r["cid2score"].items())] for r in records])
+
+
+def loader_split(path):
+    """Writes the synthetic split the loader comparison reads; returns its records."""
+    from qagnn_b200 import data as Dt
+    return Dt.synth_adj_pickle(path, LOADER_CASE["n_records"], seed=LOADER_CASE["seed"])
+
+
+def batch_generator_inputs(path):
+    """Inputs of the batch-generator comparison: 10 questions x 5 choices of a synthetic split, batch size 4 (a partial last
+    batch).  Returns the generator's positional and keyword arguments (adj_data excluded) and the nested adjacency."""
+    from qagnn_b200 import data as Dt
+    n, nc, bs = 40, 5, 4
+    Dt.synth_adj_pickle(path, 50, seed=2, max_nodes=60)
+    cids, ntypes, scores, lens, (ei, et) = Dt.load_sparse_adj_data_with_contextnode(path, n, nc, None, use_cache=False,
+                                                                                   write_cache=False)
+    Q = cids.size(0)
+    qids = [f"q{i}" for i in range(Q)]
+    labels = torch.arange(Q) % nc
+    lm = torch.arange(Q * nc * 7).view(Q, nc, 7)
+    indexes = torch.randperm(Q, generator=torch.Generator().manual_seed(0))
+
+    class Args:
+        drop_partial_batch = False
+        fill_partial_batch = False
+    return dict(n=n, bs=bs, Q=Q, args=(Args(), "eval", "cpu", "cpu", bs, indexes, qids, labels),
+                kw=dict(tensors0=[lm], tensors1=[cids, ntypes, scores, lens]), ei=ei, et=et)
+
+
+def batch_generator_input_digest(case):
+    return digest([case["args"][5:], case["kw"]["tensors0"], case["kw"]["tensors1"], case["ei"], case["et"]])
+
+
+def fuzz_sample_index(numel, seed):
+    """Flat indices of the entries of a compared tensor that FUZZ_FILE keeps (all of them for small tensors)."""
+    if numel <= FUZZ_SAMPLES:
+        return torch.arange(numel)
+    return torch.randperm(numel, generator=torch.Generator().manual_seed(seed))[:FUZZ_SAMPLES].sort().values
+
+
+def fuzz_check_stored(stored, samples, tol_abs=FUZZ_TOL[0], tol_rel=FUZZ_TOL[1]):
+    """The oracle against one stored fuzz case (`samples`: FUZZ_FILE's flat tensor of sampled entries): the sampled entries
+    within `tol_abs + tol_rel*|ref|`, and every tensor's sum within the sum of those bounds (which the element-wise bound
+    implies).  Returns the worst excess; <= 0 passes."""
+    in_fp, w_fp, got = fuzz_oracle(stored["case"])
+    assert in_fp == stored["input_fp"] and w_fp == stored["weight_fp"], "regenerated fuzz inputs differ from the recorded ones"
+    assert sorted(got) == sorted(stored["tensors"]), "compared tensors differ from the recorded ones"
+    worst = -tol_abs
+    for i, (name, want) in enumerate(sorted(stored["tensors"].items())):
+        a = got[name].detach().double()
+        assert tuple(a.shape) == want["shape"], name
+        idx = fuzz_sample_index(a.numel(), stored["case"]["seed"] * 16 + i)
+        sample = samples[want["offset"]:want["offset"] + idx.numel()].double()
+        worst = max(worst, _excess(a.reshape(-1)[idx], sample, tol_abs, tol_rel))
+        worst = max(worst, abs(float(a.sum()) - want["sum"]) - a.numel() * tol_abs - tol_rel * want["abs_sum"])
+    return worst
+
+
+def record():
+    """Runs the reference where the tests compare against it and stores what it produced: DIGEST_FILE (every committed
+    fixture re-minted in memory; the reference's adjacency loader and batch generator) and FUZZ_FILE."""
+    import pickle
+    import tempfile
+    from oracle.ref_shim import load_reference_data_utils
+    torch.set_num_threads(8)
+    ref = load_reference()
+    RD = load_reference_data_utils()
+    out = {"fixtures": {case["name"]: digest(mint(ref, case)) for mint, case in all_cases()}, "loader": {}}
+    with tempfile.TemporaryDirectory() as tmp:
+        for max_node_num in (200, 30):
+            path = os.path.join(tmp, f"n{max_node_num}", "dev.graph.adj.pk")
+            os.makedirs(os.path.dirname(path))
+            records = loader_split(path)
+            res = RD.load_sparse_adj_data_with_contextnode(path, max_node_num, LOADER_CASE["num_choice"], None)
+            with open(path + ".loaded_cache", "rb") as f:
+                cache = pickle.load(f)
+            entry = {"input": records_digest(records), "cache": digest(cache)}
+            entry.update({name: digest(v) for name, v in zip(LOADER_FIELDS, res[:4] + tuple(res[4]))})
+            out["loader"][str(max_node_num)] = entry
+        case = batch_generator_inputs(os.path.join(tmp, "s.graph.adj.pk"))
+        batches = RD.MultiGPUSparseAdjDataBatchGenerator(*case["args"], adj_data=(case["ei"], case["et"]), **case["kw"])
+        out["batch_generator"] = {"input": batch_generator_input_digest(case), "batches": [digest(b) for b in batches]}
+    with open(DIGEST_FILE, "w") as f:
+        json.dump(out, f, indent=1, sort_keys=True)
+        f.write("\n")
+    cases, samples, offset = [], [], 0
+    for case in fuzz_cases(FUZZ_COUNT):
+        fx = mint_mp_case(ref, case, 4, case["n_etype"])
+        tensors = {}
+        for i, (name, t) in enumerate(sorted(_fuzz_compared(fx).items())):
+            t = t.detach().double()
+            idx = fuzz_sample_index(t.numel(), case["seed"] * 16 + i)
+            samples.append(t.reshape(-1)[idx].float())
+            tensors[name] = {"shape": tuple(t.shape), "offset": offset, "sum": float(t.sum()), "abs_sum": float(t.abs().sum())}
+            offset += idx.numel()
+        cases.append({"case": case, "input_fp": fx["input_fp"], "weight_fp": fx["weight_fp"], "tensors": tensors})
+    torch.save({"kind": "mp_fuzz", "tol": FUZZ_TOL, "cases": cases, "samples": torch.cat(samples)}, FUZZ_FILE)
+
+
+def reference_digests():
+    with open(DIGEST_FILE) as f:
+        return json.load(f)
+
+
 def main():
+    if "--record" in sys.argv[1:]:
+        record()
+        print("wrote", DIGEST_FILE, "and", FUZZ_FILE)
+        return
     if "--fuzz" in sys.argv[1:]:
         count = int(sys.argv[sys.argv.index("--fuzz") + 1])
         bad = 0

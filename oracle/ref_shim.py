@@ -17,8 +17,8 @@ This shim registers stand-ins for exactly the third-party entry points the hot p
 restated from their published semantics (SURVEY.md §8 rows a6-a8).  Everything under
 /root/reference then runs verbatim.
 
-Only `oracle/make_goldens.py` and tests that are skipped when /root/reference is absent
-may import this file.
+Only `oracle/make_goldens.py` calls into this file; the tests read what it recorded under
+tests/golden/ and never need the reference tree.
 """
 import inspect
 import os
@@ -174,3 +174,14 @@ def load_reference():
     import importlib
     _REF = importlib.import_module("modeling.modeling_qagnn")
     return _REF
+
+
+def load_reference_data_utils():
+    """Returns the reference's `utils.data_utils` module (adjacency loader and batch generator, imported verbatim)."""
+    if not os.path.isfile(os.path.join(REFERENCE_ROOT, "utils", "data_utils.py")):
+        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+    _install_stubs()
+    if REFERENCE_ROOT not in sys.path:
+        sys.path.insert(0, REFERENCE_ROOT)
+    import importlib
+    return importlib.import_module("utils.data_utils")

@@ -95,3 +95,23 @@ def test_committed_bench_lines_are_self_consistent(name):
     assert not set(d["clocks"]["reasons"]) & {"hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown"}
     if G > 1:
         assert d["parity_gate"]["multi_rank_logits_vs_single_gpu_max_abs_err"] < 1e-5
+
+
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]])
+def test_bad_arguments_are_refused(extra):
+    """--steps is the number of timed steps (at least one); --dump-outputs belongs to the CUDA arm, whose inputs are seeded."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                         cwd=ROOT)
+    assert out.returncode == 2 and "error:" in out.stderr
+    assert not os.path.exists(os.path.join(ROOT, "unused"))
+
+
+def test_dump_outputs_writes_float32_npy_within_the_limit(tmp_path):
+    import numpy as np
+    import bench
+    bench.dump_outputs(str(tmp_path / "d"), {"a": np.arange(6.0).reshape(2, 3)})
+    got = np.load(tmp_path / "d" / "a.npy")
+    assert got.dtype == np.float32 and got.tolist() == [[0, 1, 2], [3, 4, 5]]
+    with pytest.raises(SystemExit):
+        bench.dump_outputs(str(tmp_path / "e"), {"big": np.zeros(bench.DUMP_LIMIT // 4 + 1, np.float32)})
+    assert not (tmp_path / "e").exists()

@@ -1,15 +1,14 @@
 """The adjacency loader keeps the reference's input format (utils/data_utils.py:79-197): checked field by field
-against the reference's own loader when /root/reference is present (build container), and always against its
+against what the reference's own loader and batch generator produced (content digests in
+tests/golden/reference_digests.json, recorded by `python -m oracle.make_goldens --record`), and against its
 structural invariants."""
-import os
-import sys
+import pickle
 
 import pytest
 import torch
 
+from oracle import make_goldens as MG
 from qagnn_b200 import data as Dt
-
-REF = "/root/reference"
 
 
 def _equal_nested(a, b):
@@ -18,25 +17,19 @@ def _equal_nested(a, b):
 
 @pytest.mark.parametrize("max_node_num", [200, 30])
 def test_loader_matches_reference_loader(tmp_path, max_node_num):
-    if not os.path.isdir(os.path.join(REF, "utils")):
-        pytest.skip("reference tree not available (GPU box)")
+    want = MG.reference_digests()["loader"][str(max_node_num)]
     path = str(tmp_path / "dev.graph.adj.pk")
-    Dt.synth_adj_pickle(path, 20, seed=4)
-    ours = Dt.load_sparse_adj_data_with_contextnode(path, max_node_num, 5, None, use_cache=False, write_cache=False)
-    sys.path.insert(0, REF)
-    try:
-        from oracle.ref_shim import _install_stubs
-        _install_stubs()
-        from utils import data_utils as RD
-        ref = RD.load_sparse_adj_data_with_contextnode(path, max_node_num, 5, None)
-    finally:
-        sys.path.remove(REF)
-    for a, b, name in zip(ours[:4], ref[:4], ("concept_ids", "node_type_ids", "node_scores", "adj_lengths")):
-        assert a.dtype == b.dtype and torch.equal(a, b), name
-    assert _equal_nested(ours[4][0], ref[4][0]) and _equal_nested(ours[4][1], ref[4][1])
-    # the cache the reference just wrote is readable by our loader and gives the same answer
+    records = MG.loader_split(path)
+    assert MG.records_digest(records) == want["input"], "the synthetic split differs from the one the reference loaded"
+    ours = Dt.load_sparse_adj_data_with_contextnode(path, max_node_num, 5, None, use_cache=False, write_cache=True)
+    for name, value in zip(MG.LOADER_FIELDS, ours[:4] + ours[4]):
+        assert MG.digest(value) == want[name], name
+    # the cache next to the split is the reference's `.loaded_cache`, item for item, and reading it gives the same answer
+    with open(path + ".loaded_cache", "rb") as f:
+        assert MG.digest(pickle.load(f)) == want["cache"]
     cached = Dt.load_sparse_adj_data_with_contextnode(path, max_node_num, 5, None, use_cache=True)
-    assert torch.equal(cached[0], ref[0]) and _equal_nested(cached[4][0], ref[4][0])
+    for name, value in zip(MG.LOADER_FIELDS, cached[:4] + cached[4]):
+        assert MG.digest(value) == want[name], name
 
 
 def test_loader_invariants_and_packing(tmp_path):
@@ -106,41 +99,22 @@ def test_flat_cache_answers_what_the_reference_dataloader_asks_of_adj_data(tmp_p
 
 
 def test_packed_batch_generator_matches_reference_generator(tmp_path):
-    n, nc, bs = 40, 5, 4
-    path, (cids, ntypes, scores, lens, (ei, et)) = _make_split(tmp_path, 50, n, nc)  # 10 questions
-    Q = cids.size(0)
-    qids = [f"q{i}" for i in range(Q)]
-    labels = torch.arange(Q) % nc
-    lm = torch.arange(Q * nc * 7).view(Q, nc, 7)
-    indexes = torch.randperm(Q, generator=torch.Generator().manual_seed(0))
-
-    class Args:
-        drop_partial_batch = False
-        fill_partial_batch = False
-    kw = dict(tensors0=[lm], tensors1=[cids, ntypes, scores, lens])
+    want = MG.reference_digests()["batch_generator"]
+    case = MG.batch_generator_inputs(str(tmp_path / "s.graph.adj.pk"))
+    assert MG.batch_generator_input_digest(case) == want["input"], "the inputs differ from the ones the reference batched"
+    n, bs, Q, ei, et = case["n"], case["bs"], case["Q"], case["ei"], case["et"]
     flat = Dt.FlatAdjCache.from_nested(ei, et, n)
-    ours = list(Dt.PackedAdjBatchGenerator(Args(), "eval", "cpu", "cpu", bs, indexes, qids, labels, adj_data=flat, **kw))
-    nested = list(Dt.PackedAdjBatchGenerator(Args(), "eval", "cpu", "cpu", bs, indexes, qids, labels, adj_data=(ei, et), **kw))
-    ref = nested
-    if os.path.isdir(os.path.join(REF, "utils")):  # build container: the reference's own generator
-        sys.path.insert(0, REF)
-        try:
-            from oracle.ref_shim import _install_stubs
-            _install_stubs()
-            from utils import data_utils as RD
-            ref = list(RD.MultiGPUSparseAdjDataBatchGenerator(Args(), "eval", "cpu", "cpu", bs, indexes, qids, labels,
-                                                              adj_data=(ei, et), **kw))
-        finally:
-            sys.path.remove(REF)
-    assert len(ours) == len(ref) == len(nested) == (Q + bs - 1) // bs
-    for bo, bn, br in zip(ours, nested, ref):
-        assert bo[0] == br[0] == bn[0] and torch.equal(bo[1], br[1])
-        for x, y, z in zip(bo[2:-2], br[2:-2], bn[2:-2]):
-            assert torch.equal(x, y) and torch.equal(z, y)
-        assert _equal_nested(bn[-2], br[-2]) and _equal_nested(bn[-1], br[-1])
-        want = Dt.pack_adj(br[-2], br[-1], n, pin=False)  # == LM_QAGNN.batch_graph of the reference's nested batch
+    ours = list(Dt.PackedAdjBatchGenerator(*case["args"], adj_data=flat, **case["kw"]))
+    nested = list(Dt.PackedAdjBatchGenerator(*case["args"], adj_data=(ei, et), **case["kw"]))
+    assert len(ours) == len(nested) == len(want["batches"]) == (Q + bs - 1) // bs
+    for bo, bn, wd in zip(ours, nested, want["batches"]):
+        assert MG.digest(bn) == wd  # the nested batch is the reference's MultiGPUSparseAdjDataBatchGenerator batch
+        assert bo[0] == bn[0] and torch.equal(bo[1], bn[1])
+        for x, z in zip(bo[2:-2], bn[2:-2]):
+            assert torch.equal(x, z)
+        want_packed = Dt.pack_adj(bn[-2], bn[-1], n, pin=False)  # == LM_QAGNN.batch_graph of the reference's nested batch
         assert isinstance(bo[-2], Dt.PackedAdj)
-        assert torch.equal(bo[-2].edge_index, want.edge_index) and torch.equal(bo[-1], want.edge_type)
+        assert torch.equal(bo[-2].edge_index, want_packed.edge_index) and torch.equal(bo[-1], want_packed.edge_type)
 
 
 def _batches_equal(a, b):
