@@ -237,6 +237,9 @@ bool use_slice(const qagnn_shape& s) {
   const char* e = getenv("QAGNN_MP_PATH");
   return !(e && strcmp(e, "basic") == 0) && slice_supported(s);
 }
+// Some message-passing path takes the shape.  Checked at the entry points before anything is launched: a width no path
+// can run (D % 4 != 0 without per-graph tiles) is refused up front instead of after the projection GEMM.
+bool mp_path_supported(const qagnn_shape& s) { return use_headtile(s) || use_slice(s) || basic_mp_supported(s); }
 
 // one GATConvE layer; `final_act` = ACT_NONE for the bare layer, ACT_GELU when called from mp_helper
 int32_t layer_forward(const qagnn_shape& s, const FoldLayout& L, const WorkLayout& W, int layer, const float* x,
@@ -441,6 +444,7 @@ extern "C" int32_t qagnn_gatconve_forward(const qagnn_shape* shape, int32_t laye
   QAGNN_RETURN_IF(check_shape_fwd(shape));
   if (!x || !extra || !prep || !folded || !out || !workspace) return QAGNN_ERR_INVALID_ARGUMENT;
   if (layer < 0 || layer >= shape->k) return QAGNN_ERR_INVALID_ARGUMENT;
+  if (!mp_path_supported(*shape)) return QAGNN_ERR_UNSUPPORTED;
   const FoldLayout L = make_fold_layout(*shape);
   const WorkLayout W = make_work_layout(*shape);
   if (workspace_bytes < W.total * sizeof(float)) return QAGNN_ERR_WORKSPACE;
@@ -479,6 +483,7 @@ extern "C" int32_t qagnn_mp_forward(const qagnn_shape* shape, const float* H_in,
   QAGNN_RETURN_IF(check_shape_fwd(shape));
   if (!H_in || !node_type || !node_score || !prep || !folded || !out || !workspace) return QAGNN_ERR_INVALID_ARGUMENT;
   const qagnn_shape& s = *shape;
+  if (s.k > 0 && !mp_path_supported(s)) return QAGNN_ERR_UNSUPPORTED;
   const FoldLayout L = make_fold_layout(s);
   const WorkLayout W = make_work_layout(s);
   if (workspace_bytes < W.total * sizeof(float)) return QAGNN_ERR_WORKSPACE;

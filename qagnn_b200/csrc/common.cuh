@@ -165,6 +165,9 @@ int32_t launch_message_passing_headtile(const qagnn_shape& s, const int32_t* pre
                                         cudaStream_t st);
 int32_t zero_head_pads(const qagnn_shape& s, float* qkmh, cudaStream_t st);
 
+// the general CSR kernels (message_passing.cu) and their backward (mp_backward.cu) are instantiated for these shapes:
+// D % 4 == 0 (float4 columns), D <= 1024 (8 chunks per lane), H in {1, 2, 4, 8, 16}
+bool basic_mp_supported(const qagnn_shape& s);
 int32_t launch_message_passing(const qagnn_shape& s, const int32_t* prep_base, const qagnn_prep_layout& pl,
                                const float* qkm, const float* ke, const float* me, float* score, float* alpha,
                                float* aggr, float* alpha_out, cudaStream_t st);

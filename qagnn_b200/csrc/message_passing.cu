@@ -214,10 +214,14 @@ int32_t launch_h(const qagnn_shape& s, const int32_t* base, const qagnn_prep_lay
 
 }  // namespace
 
+bool basic_mp_supported(const qagnn_shape& s) {
+  return s.D % 4 == 0 && s.D <= 1024 && (s.H == 1 || s.H == 2 || s.H == 4 || s.H == 8 || s.H == 16);
+}
+
 int32_t launch_message_passing(const qagnn_shape& s, const int32_t* prep_base, const qagnn_prep_layout& pl,
                                const float* qkm, const float* ke, const float* me, float* score, float* alpha,
                                float* aggr, float* alpha_out, cudaStream_t st) {
-  if (s.D % 4 != 0 || s.D > 1024) return QAGNN_ERR_UNSUPPORTED;
+  if (!basic_mp_supported(s)) return QAGNN_ERR_UNSUPPORTED;
   switch (s.H) {
     case 1: return launch_h<1>(s, prep_base, pl, qkm, ke, me, score, alpha, aggr, alpha_out, st);
     case 2: return launch_h<2>(s, prep_base, pl, qkm, ke, me, score, alpha, aggr, alpha_out, st);

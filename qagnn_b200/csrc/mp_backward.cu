@@ -314,12 +314,13 @@ int32_t launch_message_passing_backward(const qagnn_shape& s, const int32_t* pre
                                         const int32_t* combo_order, const float* qkm, const float* ke, const float* me,
                                         const float* alpha_s, const float* d_aggr, float* ds, float* d_qkm, float* d_ke,
                                         float* d_me, cudaStream_t st) {
-  if (s.D % 4 != 0 || s.D > 1024) return QAGNN_ERR_UNSUPPORTED;
+  if (!basic_mp_supported(s)) return QAGNN_ERR_UNSUPPORTED;
   switch (s.H) {
     case 1: return launch_bwd_h<1>(s, prep_base, pl, combo_order, qkm, ke, me, alpha_s, d_aggr, ds, d_qkm, d_ke, d_me, st);
     case 2: return launch_bwd_h<2>(s, prep_base, pl, combo_order, qkm, ke, me, alpha_s, d_aggr, ds, d_qkm, d_ke, d_me, st);
     case 4: return launch_bwd_h<4>(s, prep_base, pl, combo_order, qkm, ke, me, alpha_s, d_aggr, ds, d_qkm, d_ke, d_me, st);
     case 8: return launch_bwd_h<8>(s, prep_base, pl, combo_order, qkm, ke, me, alpha_s, d_aggr, ds, d_qkm, d_ke, d_me, st);
+    case 16: return launch_bwd_h<16>(s, prep_base, pl, combo_order, qkm, ke, me, alpha_s, d_aggr, ds, d_qkm, d_ke, d_me, st);
     default: return QAGNN_ERR_UNSUPPORTED;
   }
 }

@@ -41,6 +41,29 @@ def assert_close(got, ref, what="", atol=ATOL, rtol=RTOL):
     return err.max().item() if err.numel() else 0.0
 
 
+def mp_core_reference(qkm, ke, me, prep, H):
+    """The graph part of one GATConvE layer on node-level projections — what `training._MPCore` computes — restated in
+    vectorised torch ops in the dtype of the inputs (fp64 in the tests), differentiable by autograd:
+
+        s[e,h]  = Q[src] . (Kx[tgt] + Ke[combo])       per head, over the d = D/H columns of head h
+        a       = softmax of s over the edges that share SRC          a' = a * outdeg(src)
+        aggr[v] = sum_{e: tgt = v} a'[e,h] (Mx[src] + Me[combo])
+
+    qkm [N, 3D] = Q | Kx | Mx; ke, me [C, D]; `prep` = O.graph_prep_oracle(...) (edges then self loops).
+    Returns (aggr [N, D], alpha [E+N, H]) with alpha before the out-degree rescale, in edge_index' order."""
+    N, D = qkm.size(0), qkm.size(1) // 3
+    d = D // H
+    src, tgt, combo = (torch.from_numpy(prep[k]) for k in ("src", "tgt", "combo"))
+    outdeg = torch.from_numpy(prep["outdeg"]).to(qkm.dtype)
+    Q, Kx, Mx = (qkm[:, i * D:(i + 1) * D].reshape(N, H, d) for i in range(3))
+    Ke, Me = ke.reshape(-1, H, d), me.reshape(-1, H, d)
+    s = (Q[src] * (Kx[tgt] + Ke[combo])).sum(-1)
+    a = O.segment_softmax(s, src)
+    a_scaled = a * outdeg[src][:, None]
+    aggr = O.scatter_sum(a_scaled[:, :, None] * (Mx[src] + Me[combo]), tgt, N)
+    return aggr.reshape(N, D), a
+
+
 def regen_mp_inputs(fx):
     c = fx["case"]
     inp = O.synth_graph_batch(c["B"], c["n"], c["e"], c["D"], fx["n_etype"], c["seed"], c["realistic"])

@@ -76,7 +76,7 @@ def _factorised_layer(sd, prefix, x, score_emb, type_emb_rows, nt, prep, T, R, H
     aggr = aggr.view(N, D)
     W1, b1 = _fold_bn(sd, prefix + ".mlp.0", prefix + ".mlp.1")
     out = torch.relu(aggr @ W1.t() + b1) @ sd[prefix + ".mlp.3.weight"].to(F64).t() + sd[prefix + ".mlp.3.bias"].to(F64)
-    return out, a, aggr
+    return out, a, aggr, (qkm, Ke, Me)
 
 
 def _factorised_forward(sd, b, k, T, R, H):
@@ -90,32 +90,53 @@ def _factorised_forward(sd, b, k, T, R, H):
     X = b["H"].to(F64).reshape(-1, D)
     layers = []
     for l in range(k):
-        X, a, aggr = _factorised_layer(sd, f"gnn_layers.{l}", X, score_emb, type_emb_rows, nt, prep, T, R, H)
+        X, a, aggr, proj = _factorised_layer(sd, f"gnn_layers.{l}", X, score_emb, type_emb_rows, nt, prep, T, R, H)
         X = O.gelu_tanh(X)
-        layers.append({"x": X, "alpha": a, "aggr": aggr})
+        layers.append({"x": X, "alpha": a, "aggr": aggr, "proj": proj})
     Vcat = torch.cat([sd["Vh.weight"], sd["Vx.weight"]], dim=1).to(F64)     # one GEMM over [H | X]
     out = O.gelu_tanh(torch.cat([b["H"].to(F64).reshape(-1, D), X], dim=1) @ Vcat.t() + (sd["Vh.bias"].to(F64) + sd["Vx.bias"].to(F64)))
-    return out.view(Bn, n, D), layers
+    return out.view(Bn, n, D), layers, prep
 
 
-@pytest.mark.parametrize("regime,realistic,B,n,e,D,H,k,R", [
+_FACTORISATION_CASES = [
     ("peaky", False, 3, 12, 40, 16, 4, 2, 38),
     ("prod", True, 4, 20, 60, 24, 4, 3, 38),
     ("peaky", True, 2, 9, 0, 16, 2, 1, 6),       # no real edges: self loops only
     ("peaky", False, 1, 1, 3, 8, 2, 2, 5),       # one node, three i->i edges
-])
+]
+
+
+@pytest.mark.parametrize("regime,realistic,B,n,e,D,H,k,R", _FACTORISATION_CASES)
 def test_node_level_factorisation_equals_the_per_edge_form(regime, realistic, B, n, e, D, H, k, R):
     T = 4
     b = O.synth_graph_batch(B, n, e, D, n_etype=R, seed=11, realistic=realistic)
     sd = O.random_state_dict(k, D, T, R, regime=regime, seed=3)
     want, _, want_layers = O.message_passing_forward(sd, b["H"], b["edge_index"], b["edge_type"], b["node_type"], b["node_score"],
                                                     k, T, R, head_count=H, dtype=F64, return_layers=True)
-    got, got_layers = _factorised_forward(sd, b, k, T, R, H)
+    got, got_layers, _ = _factorised_forward(sd, b, k, T, R, H)
     for g, w in zip(got_layers, want_layers):
         assert torch.allclose(g["alpha"], w["alpha"], rtol=0, atol=1e-12)
         assert torch.allclose(g["aggr"], w["aggr"], rtol=1e-10, atol=1e-10)
         assert torch.allclose(g["x"], w["x"], rtol=1e-10, atol=1e-10)
     assert torch.allclose(got, want, rtol=1e-10, atol=1e-10)
+
+
+@pytest.mark.parametrize("regime,realistic,B,n,e,D,H,k,R", _FACTORISATION_CASES)
+def test_mp_core_reference_on_factorised_projections_equals_the_per_edge_form(regime, realistic, B, n, e, D, H, k, R):
+    """tests/helpers.mp_core_reference — the fp64 reference the GPU kernel tests compare _MPCore with — fed the factorised
+    Q|Kx|Mx, Ke, Me of every layer gives the oracle's per-edge alpha and aggr."""
+    from tests import helpers as Hh
+    T = 4
+    b = O.synth_graph_batch(B, n, e, D, n_etype=R, seed=11, realistic=realistic)
+    sd = O.random_state_dict(k, D, T, R, regime=regime, seed=3)
+    _, _, want_layers = O.message_passing_forward(sd, b["H"], b["edge_index"], b["edge_type"], b["node_type"], b["node_score"],
+                                                  k, T, R, head_count=H, dtype=F64, return_layers=True)
+    _, got_layers, prep = _factorised_forward(sd, b, k, T, R, H)
+    for g, w in zip(got_layers, want_layers):
+        qkm, Ke, Me = g["proj"]
+        aggr, alpha = Hh.mp_core_reference(qkm, Ke, Me, prep, H)
+        assert torch.allclose(alpha, w["alpha"], rtol=1e-10, atol=1e-10)
+        assert torch.allclose(aggr, w["aggr"], rtol=1e-10, atol=1e-10)
 
 
 def _mp(sd, b, k, R, H=4, **kw):

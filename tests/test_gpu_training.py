@@ -97,24 +97,40 @@ def test_dropout_is_applied_in_training_mode_only():
     assert torch.equal(e1, e2) and float((e1 == 0).float().mean()) < 0.01
 
 
-def test_single_layer_training_gradients_against_autograd_of_the_oracle():
-    """GATConvE alone in .train(): gradients of x / extra / weights vs autograd through the CPU oracle's op-for-op
-    restatement with batch statistics (the oracle is differentiable: it is written in torch ops)."""
+def _hub_graph_batch(D, seed):
+    """One 200-node graph in which node 3 is the source of 600 edges and node 8 the target of 600 more."""
+    g = torch.Generator().manual_seed(seed)
+    n = 200
+    ei = torch.randint(0, n, (2, 1400), generator=g)
+    ei[0, :600] = 3
+    ei[1, 600:1200] = 8
+    nt = torch.randint(0, 3, (1, n), generator=g)
+    nt[0, 0] = 3
+    return {"H": torch.randn(1, n, D, generator=g) * 0.5, "edge_index": ei, "edge_type": torch.randint(0, 38, (1400,), generator=g),
+            "node_type": nt}
+
+
+def _single_layer_training_check(D, Hd, graph):
+    """GATConvE alone in .train(): out, alpha and the gradients of x / extra / every parameter vs autograd through the CPU
+    oracle's op-for-op restatement with batch statistics, evaluated in fp64 (the oracle is differentiable: it is written in
+    torch ops)."""
     from oracle import qagnn_oracle as O
-    D, Hd, T, R = 64, 4, 4, 38
-    inp = O.synth_graph_batch(3, 30, 90, D, R, seed=31)
+    T, R = 4, 38
+    inp = O.synth_graph_batch(3, 30, 90, D, R, seed=31) if graph == "random" else _hub_graph_batch(D, seed=31)
     sd = O.random_state_dict(1, D, T, R, "peaky", seed=31)
     x = inp["H"].view(-1, D).clone().requires_grad_(True)
     g0 = torch.Generator().manual_seed(5)
     extra = (torch.randn(x.shape, generator=g0) * 0.5).requires_grad_(True)
     nt = inp["node_type"].view(-1)
+    ref_params = {k_[len("gnn_layers.0."):]: v.requires_grad_(True) for k_, v in sd.items()
+                  if k_.startswith("gnn_layers.0.") and v.is_floating_point() and "running_" not in k_}
     ref_out, _, ref_alpha, _ = O.gatconve_forward(sd, "gnn_layers.0", x, inp["edge_index"], inp["edge_type"], nt, extra, T, R,
-                                                  head_count=Hd, train=True)
+                                                  head_count=Hd, dtype=torch.float64, train=True)
     G = torch.randn(ref_out.shape, generator=g0)
-    (ref_out * G).sum().backward()
+    (ref_out * G.double()).sum().backward()
     enc = torch.nn.Sequential(torch.nn.Linear(R + 1 + 2 * T, D), torch.nn.BatchNorm1d(D), torch.nn.ReLU(), torch.nn.Linear(D, D))
     layer = qagnn_b200.GATConvE(None, D, T, R, enc, head_count=Hd)
-    layer.load_state_dict({k_[len("gnn_layers.0."):]: v for k_, v in sd.items() if k_.startswith("gnn_layers.0.")})
+    layer.load_state_dict({k_[len("gnn_layers.0."):]: v.detach() for k_, v in sd.items() if k_.startswith("gnn_layers.0.")})
     layer = layer.to(DEV).train()
     xg = x.detach().to(DEV).requires_grad_(True)
     eg = extra.detach().to(DEV).requires_grad_(True)
@@ -124,6 +140,25 @@ def test_single_layer_training_gradients_against_autograd_of_the_oracle():
     (out * G.to(DEV)).sum().backward()
     _grad_close(xg.grad, x.grad, "dL/dx")
     _grad_close(eg.grad, extra.grad, "dL/dextra")
+    got = dict(layer.named_parameters())
+    assert sorted(got) == sorted(ref_params)
+    gmax = max(float(p.grad.abs().max()) for p in ref_params.values())
+    for pname, ref_p in ref_params.items():
+        # floor: the biases in front of a BatchNorm have a mathematically zero gradient (rounding noise in both)
+        _grad_close(got[pname].grad, ref_p.grad, f"dL/d{pname}", floor=1e-2 * gmax)
+
+
+def test_single_layer_training_gradients_against_autograd_of_the_oracle():
+    """D = 64, H = 4 on a batch of three random 30-node graphs."""
+    _single_layer_training_check(64, 4, "random")
+
+
+@pytest.mark.parametrize("D,Hd,graph", [(64, 1, "random"), (128, 2, "random"), (1024, 8, "random"), (256, 16, "random"),
+                                        (64, 4, "hub"), (256, 16, "hub")])
+def test_single_layer_training_gradients_at_every_head_count(D, Hd, graph):
+    """The same check at H = 1, 2, 8, 16 and on a graph with 600-edge source / target hubs: the wiring around the
+    message-passing kernels (per-head 1/sqrt(d), the node / edge halves of the key and msg weights) for every head count."""
+    _single_layer_training_check(D, Hd, graph)
 
 
 def test_whole_decoder_training_step_matches_reference():
